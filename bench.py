@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- FK + end-effector Jacobian throughput of the Kuka iiwa 7-DoF (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One *step* = one pass of the hot path (one `drmb200_fk_jacobian` launch: pos, quat, J_lin, J_ang
 of `iiwa_link_ee`) over one batch of 65 536 synthetic joint configurations (BASELINE.json
@@ -31,6 +31,10 @@ Extra keys on the JSON line (see DESIGN.md "Measurement"):
   cpu_baseline_port   the vectorised torch CPU port of the same algorithm (oracle/drm_oracle.py)
   clocks              nvidia-smi SM clocks / throttle reasons sampled during the timed regions
 
+`--dump-outputs DIR` writes what the last timed step computed on rank 0 -- pos, quat, J_lin, J_ang of its 65 536
+configurations -- as DIR/<name>.npy (float32, 12.8 MB).  The inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
+
 `--impl reference` times the reference's own CPU implementation through its public API
 (`DifferentiableRobotModel.compute_endeffector_jacobian`, unmodified, installed into baseline/_ref by
 `__graft_entry__.build()`; its third-party XML-parser dependency is replaced by oracle/refshim) --
@@ -45,6 +49,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 REPO = os.path.dirname(os.path.abspath(__file__))
@@ -284,8 +289,12 @@ def main():
     ap.add_argument("--no-large", action="store_true")
     ap.add_argument("--no-modes", action="store_true")
     ap.add_argument("--no-sharded", action="store_true", help="skip the sharded BASELINE configs 4 and 5 (scripts/bench_sharded.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (rank 0) as DIR/{pos,quat,jac_lin,jac_ang}.npy, float32")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; it does not apply to --impl reference")
 
     if args.impl == "reference":
         run_reference_arm(args)
@@ -427,6 +436,10 @@ def main():
         if sampler:
             sampler.mark_end()
         elapsed_ms = job_ms(region_ms)
+        dumped = None
+        if args.dump_outputs and rank == 0:                  # copied now: the sections below reuse these buffers
+            dumped = {name: t.cpu().numpy() for name, t in
+                      zip(("pos", "quat", "jac_lin", "jac_ang"), outs[(args.steps - 1) % ROTATE])}
 
         modes = None
         if not args.no_modes:
@@ -600,6 +613,10 @@ def main():
                     "kind": "port", "sample": "2^20 configurations through oracle/drm_oracle.c (scalar C, one pthread per core)"}
             except Exception as exc:      # the C oracle is optional context
                 result["cpu_baseline_c_port"] = {"error": str(exc)}
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         print(json.dumps(result))
     if world > 1:
         dist.destroy_process_group()

@@ -16,7 +16,7 @@ from differentiable_robot_model_b200 import engine, link_table
 from differentiable_robot_model_b200.rigid_body_params import PositiveScalar, UnconstrainedScalar, UnconstrainedTensor
 
 
-def quiet(stem, capsys=None, device=None):
+def quiet(stem, capsys=None, device="cpu"):
     return drm.DifferentiableRobotModel(urdf_path(stem), stem, device=device)
 
 
@@ -81,12 +81,13 @@ def test_wrappers_and_exports():
     for cls, n in ((drm.DifferentiableKUKAiiwa, 7), (drm.DifferentiableFrankaPanda, 7),
                    (drm.DifferentiableTwoLinkRobot, 2), (drm.DifferentiableTrifingerEdu, 9)):
         m = cls()
-        assert m._n_dofs == n and m._device.type == "cpu"
+        # the default device is the current CUDA device where there is one, the CPU (a host-side model) elsewhere
+        assert m._n_dofs == n and m._device.type == ("cuda" if torch.cuda.is_available() else "cpu")
         assert os.path.exists(m.urdf_path)
 
 
 def test_argument_validation_matches_reference_exceptions():
-    m = drm.DifferentiableKUKAiiwa()
+    m = drm.DifferentiableKUKAiiwa(device="cpu")
     with pytest.raises(AssertionError):                       # wrong DoF count (robot_model.py:153)
         m.compute_forward_kinematics(torch.zeros(3, 6), "iiwa_link_ee")
     with pytest.raises(AssertionError):                       # ndim 3 (robot_model.py:43)
@@ -103,7 +104,7 @@ def test_argument_validation_matches_reference_exceptions():
 
 def test_no_cpu_fallback():
     """The product path must fail loudly instead of computing on the CPU."""
-    m = drm.DifferentiableKUKAiiwa()
+    m = drm.DifferentiableKUKAiiwa(device="cpu")
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         m.compute_forward_kinematics(torch.zeros(3, 7), "iiwa_link_ee")
     with pytest.raises(RuntimeError, match="no CPU fallback"):
@@ -183,13 +184,16 @@ def test_c_abi_library_exports_every_declared_symbol():
     assert sorted(engine.declared_symbols()) == declared       # the Python binding covers the whole header
     lib = engine.lib()
     assert lib.drmb200_version() >= 100
-    assert lib.drmb200_launch_count() == 0                     # nothing can have launched without a GPU
+    launches = lib.drmb200_launch_count()
+    if not torch.cuda.is_available():
+        assert launches == 0                                   # nothing can have launched without a GPU
     # argument validation happens before any device work, so it can be exercised here
     topo = drm.DifferentiableKUKAiiwa()._topology
     rc = lib.drmb200_fk_jacobian(ctypes.byref(topo), 99, None, None, 4, None, None, None, None, None)
     assert rc == -1 and b"ee_link" in lib.drmb200_last_error()
     rc = lib.drmb200_inverse_dynamics(ctypes.byref(topo), None, None, None, None, -5, 3, None, None)
     assert rc == -1
+    assert lib.drmb200_launch_count() == launches              # rejected calls launch nothing
 
 
 def test_spatial_inertia_value_operations_match_the_oracle():
@@ -199,7 +203,7 @@ def test_spatial_inertia_value_operations_match_the_oracle():
     from differentiable_robot_model_b200.spatial_vector_algebra import (DifferentiableSpatialRigidBodyInertia,
                                                                          SpatialMotionVec)
     from oracle import drm_oracle as O
-    m = drm.DifferentiableKUKAiiwa()
+    m = drm.DifferentiableKUKAiiwa(device="cpu")
     robot = O.load_robot(m.urdf_path, torch.float32)
     gen = torch.Generator().manual_seed(0)
     ang, lin = torch.randn(5, 3, generator=gen), torch.randn(5, 3, generator=gen)
